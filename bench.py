@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the IQ sample-processing path on B200 (and the CPU reference arm).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...        (N > 1)
 
 Workload (BASELINE.json configs[4], per-GPU share; configs[1] and [2] are its two halves):
@@ -36,6 +36,7 @@ sys.path.insert(0, ROOT)
 
 CAPTURE_BYTES = 48_000_000          # 10 s at 2.4 MS/s
 CAPTURE_SAMPLES = CAPTURE_BYTES // 2
+DUMP_BYTES = 60_000_000             # --dump-outputs: .npy payload of all files together (64 MB with headers and margin)
 METRIC = "complex MS/s through u8->FFT-spectrum + u8->FIR->FM chains (batched 10 s captures)"
 
 
@@ -89,6 +90,24 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(directory, outputs, budget=DUMP_BYTES):
+    """Write every (name, [rows, n] float32 tensor) of `outputs` to directory/<name>.npy.  An output that does not fit
+    what is left of `budget` is cut to a fixed sample of its rows (np.random.default_rng(0), rows kept in order), so
+    runs with the same arguments write the same rows.  Returns {name: rows written}."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    written = {}
+    for name, t in outputs:
+        rows, row_bytes = t.shape[0], t[0].numel() * 4
+        keep = min(rows, budget // row_bytes)
+        idx = np.arange(rows) if keep == rows else np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+        a = t.index_select(0, torch.from_numpy(idx).to(t.device)).cpu().numpy().astype(np.float32, copy=False)
+        np.save(os.path.join(directory, name + ".npy"), a)
+        budget -= keep * row_bytes
+        written[name] = keep
+    return written
 
 
 def workload_config(B, world, fir_engine="tensor"):
@@ -295,7 +314,7 @@ def split_capture_probe(pkg, sharding, sdr, dist, torch, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every timed section")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--captures-per-gpu", type=int, default=512)
@@ -306,7 +325,13 @@ def main():
     ap.add_argument("--fir-engine", default="tensor", choices=["tensor", "fp32"],
                     help="stage-1 FIR engine of the batched WBFM chain the step (and e2e) runs: tensor = exact u8 x s8 tcgen05 product "
                          "(csrc/wbfm_tc.cuh), fp32 = CUDA-core scatter FIR (csrc/wbfm.cuh); the other engine is timed beside it")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned on rank 0 (its captures are the job's first "
+                         "captures-per-gpu) as DIR/spectrum.npy [captures, 1024] and DIR/wbfm_audio.npy [captures, 48 kHz "
+                         "samples], float32; outputs over the %d-byte budget are a fixed seeded sample of their captures" % DUMP_BYTES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -389,6 +414,9 @@ def main():
     l0 = sdr.kernel_launches()
     ms_total = timed(3, args.steps)
     launches = sdr.kernel_launches() - l0
+    if args.dump_outputs and rank == 0:   # spec / audio hold the last timed step's results until the next step runs
+        dumped = dump_outputs(args.dump_outputs, [("spectrum", spec.view(B, 1024)), ("wbfm_audio", audio.view(B, n_audio))])
+        sys.stderr.write(f"dump-outputs: captures written {dumped} to {args.dump_outputs}\n")
     ms_spec = timed(1, args.steps)
     ms_fm = timed(2, args.steps)
     # the same WBFM batch through the OTHER stage-1 FIR engine (own context, own stream), and how far its audio is from
@@ -541,7 +569,7 @@ def main():
         sdr.batch_host(pkg.CHAIN_SPECTRUM | pkg.CHAIN_WBFM, h_iq, E, CAPTURE_BYTES, spectrum=h_spec, wbfm=h_fm)
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(2, min(args.steps, 5))
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         sdr.batch_host(pkg.CHAIN_SPECTRUM | pkg.CHAIN_WBFM, h_iq, E, CAPTURE_BYTES, spectrum=h_spec, wbfm=h_fm)
     torch.cuda.synchronize()

@@ -28,3 +28,25 @@ def test_reference_arm_other_ranks_exit_quietly():
     res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],
                          capture_output=True, text=True, env=env, timeout=120)
     assert res.returncode == 0 and res.stdout.strip() == ""
+
+
+def test_dump_outputs_writes_a_fixed_bounded_sample(tmp_path):
+    """--dump-outputs: whole outputs while they fit the budget, then the same seeded rows on every run."""
+    import importlib.util
+
+    import numpy as np
+    import torch
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    small = torch.arange(6 * 4, dtype=torch.float32).view(6, 4)
+    big = torch.arange(50 * 10, dtype=torch.float32).view(50, 10)
+    for run in ("a", "b"):
+        got = bench.dump_outputs(str(tmp_path / run), [("small", small), ("big", big)], budget=6 * 16 + 12 * 40)
+        assert got == {"small": 6, "big": 12}
+    a_small, a_big = (np.load(tmp_path / "a" / f"{n}.npy") for n in ("small", "big"))
+    assert a_small.dtype == a_big.dtype == np.float32 and np.array_equal(a_small, small.numpy())
+    rows = a_big[:, 0].astype(int) // 10
+    assert a_big.shape == (12, 10) and list(rows) == sorted(set(rows)) and np.array_equal(a_big, big.numpy()[rows])
+    assert np.array_equal(a_big, np.load(tmp_path / "b" / "big.npy"))
+    assert bench.DUMP_BYTES <= 64_000_000

@@ -55,12 +55,15 @@ SCRIPT = textwrap.dedent("""
 @pytest.mark.parametrize("tool", ["memcheck", "racecheck", "synccheck"])
 def test_compute_sanitizer_clean(tool, sdr_lib, tmp_path):
     cs = shutil.which("compute-sanitizer") or "/usr/local/cuda/bin/compute-sanitizer"
-    if not os.path.exists(cs):
-        pytest.skip("compute-sanitizer not installed")
+    if not os.access(cs, os.X_OK):
+        pytest.skip("compute-sanitizer not installed or not executable by this user")
     script = tmp_path / "run.py"
     script.write_text(SCRIPT)
-    res = subprocess.run([cs, "--tool", tool, "--error-exitcode", "9", sys.executable, str(script)],
-                         capture_output=True, text=True, timeout=900)
+    try:
+        res = subprocess.run([cs, "--tool", tool, "--error-exitcode", "9", sys.executable, str(script)],
+                             capture_output=True, text=True, timeout=900)
+    except PermissionError:
+        pytest.skip("compute-sanitizer may not be executed by this user")
     tail = (res.stdout + res.stderr)[-3000:]
     assert res.returncode == 0, tail
     assert "SANITIZED_RUN_OK" in res.stdout, tail
