@@ -33,8 +33,7 @@ def build(force=False, verbose=False):
     if not force and os.path.exists(OUT) and os.path.getmtime(OUT) >= _newest_source_mtime():
         return OUT
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    extra = os.environ.get("B200_NVCC_EXTRA", "").split()  # experiment knobs, e.g. -DB200_SPEC_MINB=4
-    cmd = [nvcc] + NVCC_FLAGS + extra + ["-o", OUT] + SOURCES
+    cmd = [nvcc] + NVCC_FLAGS + ["-o", OUT] + SOURCES
     res = subprocess.run(cmd, capture_output=True, text=True)
     log = res.stdout + res.stderr
     with open(os.path.join(HERE, "build.log"), "w") as fh:

@@ -106,33 +106,29 @@ B200_DEV void b200_am_scatter(c2 x, c2 acc0, const float (&g)[40], c2 (&acc)[4],
         acc[i & 3] = c2_fma_s(x, g[k < 40 ? k : 79 - k], acc[i & 3]);
     }
     if (J % 20 == 0 && J / 20 < B200_AM_OPT) {
-#if B200_FIR_RAWU8
         head[J / 20] = (J / 20 >= 4) ? c2_add(acc[(J / 20) & 3], acc0) : acc[(J / 20) & 3]; /* see wbfm.cuh */
-#else
-        head[J / 20] = acc[(J / 20) & 3];
-#endif
         acc[(J / 20) & 3] = acc0; /* output J/20 + 4 starts here */
     }
 }
 template <int Q>
 struct b200_am_words {
-    B200_DEVM static void run(const uint4 *raw, cvt_k cb, c2 acc0, const float (&g)[40], c2 (&acc)[4], c2 (&head)[B200_AM_OPT])
+    B200_DEVM static void run(const uint4 *raw, c2 acc0, const float (&g)[40], c2 (&acc)[4], c2 (&head)[B200_AM_OPT])
     {
         const uint4 r = raw[Q];
-        b200_am_scatter<8 * Q + 0>(B200_FIR_X_LO(r.x, cb), acc0, g, acc, head);
-        b200_am_scatter<8 * Q + 1>(B200_FIR_X_HI(r.x, cb), acc0, g, acc, head);
-        b200_am_scatter<8 * Q + 2>(B200_FIR_X_LO(r.y, cb), acc0, g, acc, head);
-        b200_am_scatter<8 * Q + 3>(B200_FIR_X_HI(r.y, cb), acc0, g, acc, head);
-        b200_am_scatter<8 * Q + 4>(B200_FIR_X_LO(r.z, cb), acc0, g, acc, head);
-        b200_am_scatter<8 * Q + 5>(B200_FIR_X_HI(r.z, cb), acc0, g, acc, head);
-        b200_am_scatter<8 * Q + 6>(B200_FIR_X_LO(r.w, cb), acc0, g, acc, head);
-        b200_am_scatter<8 * Q + 7>(B200_FIR_X_HI(r.w, cb), acc0, g, acc, head);
-        b200_am_words<Q + 1>::run(raw, cb, acc0, g, acc, head);
+        b200_am_scatter<8 * Q + 0>(c2_u8raw_lo(r.x), acc0, g, acc, head);
+        b200_am_scatter<8 * Q + 1>(c2_u8raw_hi(r.x), acc0, g, acc, head);
+        b200_am_scatter<8 * Q + 2>(c2_u8raw_lo(r.y), acc0, g, acc, head);
+        b200_am_scatter<8 * Q + 3>(c2_u8raw_hi(r.y), acc0, g, acc, head);
+        b200_am_scatter<8 * Q + 4>(c2_u8raw_lo(r.z), acc0, g, acc, head);
+        b200_am_scatter<8 * Q + 5>(c2_u8raw_hi(r.z), acc0, g, acc, head);
+        b200_am_scatter<8 * Q + 6>(c2_u8raw_lo(r.w), acc0, g, acc, head);
+        b200_am_scatter<8 * Q + 7>(c2_u8raw_hi(r.w), acc0, g, acc, head);
+        b200_am_words<Q + 1>::run(raw, acc0, g, acc, head);
     }
 };
 template <>
 struct b200_am_words<B200_AM_CHUNK / 8> {
-    B200_DEVM static void run(const uint4 *, cvt_k, c2, const float (&)[40], c2 (&)[4], c2 (&)[B200_AM_OPT]) {}
+    B200_DEVM static void run(const uint4 *, c2, const float (&)[40], c2 (&)[4], c2 (&)[B200_AM_OPT]) {}
 };
 
 __global__ void __launch_bounds__(B200_AM_THREADS, 3) k_am_front(AmFrontParams p)
@@ -144,7 +140,6 @@ __global__ void __launch_bounds__(B200_AM_THREADS, 3) k_am_front(AmFrontParams p
     c2 *s_carry = reinterpret_cast<c2 *>(smem + B200_AM_SM_CARRY);
     c2 *s_tailc = reinterpret_cast<c2 *>(smem + B200_AM_SM_TAILC);
     uint64_t *s_bar = reinterpret_cast<uint64_t *>(smem + B200_AM_SM_BAR);
-    uint32_t *s_cvt = reinterpret_cast<uint32_t *>(smem + B200_AM_SM_BAR + 8); /* conversion constants (cplx2.cuh) */
 
     const int tid = (int)threadIdx.x;
     const uint32_t capture = blockIdx.y, seg = blockIdx.x;
@@ -158,22 +153,15 @@ __global__ void __launch_bounds__(B200_AM_THREADS, 3) k_am_front(AmFrontParams p
 
     float g[40];
 #pragma unroll
-#if B200_FIR_RAWU8
     for (int k = 0; k < 40; ++k) g[k] = taps->g1s[k];
     const c2 acc0 = c2_make(taps->bias_half, taps->bias_half);
-#else
-    for (int k = 0; k < 40; ++k) g[k] = taps->g1[k];
-    const c2 acc0 = c2_zero();
-#endif
 
     /* segment 0 continues the stream exactly; later segments rebuild the FIR state from one pre-roll tile */
     const AmFrontState *st_in = (p.state && seg == 0) ? p.state + capture : nullptr;
     if (tid < 4) {
         float tr = 0.0f, ti = 0.0f;
         if (st_in) { tr = st_in->tail[2 * tid]; ti = st_in->tail[2 * tid + 1]; }
-#if B200_FIR_RAWU8
         if (seg == 0 && p.q_base == 0) tr = ti = taps->bias_head[tid]; /* first outputs of a capture / stream */
-#endif
         s_tailc[4 + tid] = c2_make(tr, ti);
     }
     for (int i = tid; i < B200_AM_NP * 12; i += B200_AM_THREADS) {
@@ -195,10 +183,8 @@ __global__ void __launch_bounds__(B200_AM_THREADS, 3) k_am_front(AmFrontParams p
         b200_mbar_init(s_bar, 1);
         b200_mbar_fence_init();
         if (my_tiles > 0) issue_tile(0);
-        b200_cvt_consts_store(s_cvt);
     }
     __syncthreads();
-    const cvt_k cb = b200_cvt_consts_load(s_cvt);
 
     for (uint32_t it = 0; it < my_tiles; ++it) {
         const uint32_t tile = t_begin + it;
@@ -213,7 +199,7 @@ __global__ void __launch_bounds__(B200_AM_THREADS, 3) k_am_front(AmFrontParams p
 #pragma unroll
         for (int i = 0; i < 4; ++i) acc[i] = start;
         const uint4 *raw = reinterpret_cast<const uint4 *>(smem + B200_AM_SM_RAW + tid * (2 * B200_AM_CHUNK));
-        b200_am_words<0>::run(raw, cb, acc0, g, acc, head);
+        b200_am_words<0>::run(raw, acc0, g, acc, head);
         if (tid == last) {
 #pragma unroll
             for (int i = 10; i < 14; ++i) s_tailc[par * 4 + (i - 10)] = acc[i & 3];

@@ -30,20 +30,7 @@ namespace {
 
 constexpr uint64_t kStreamSlack = 16384;     /* device stream buffer = ring_slots x slot_bytes + this; the unread
                                                 tail carried over a wrap is < 2048 + 400 bytes           */
-constexpr uint64_t kWaveBytesDefault = 192ull << 20;
-/* measurement knobs (tools/e2e_multi_probe.py), not part of the ABI: B200SDR_WAVE_MB overrides the wave size of
- * b200sdr_batch_host, B200SDR_PINNED_WC=1 makes b200sdr_host_alloc_pinned write-combined */
-uint64_t wave_bytes_target()
-{
-    const char *e = getenv("B200SDR_WAVE_MB");
-    const long mb = e ? atol(e) : 0;
-    return mb > 0 ? (uint64_t)mb << 20 : kWaveBytesDefault;
-}
-unsigned pinned_flags()
-{
-    const char *e = getenv("B200SDR_PINNED_WC");
-    return (e && e[0] == '1') ? cudaHostAllocWriteCombined : cudaHostAllocDefault;
-}
+constexpr uint64_t kWaveBytes = 192ull << 20; /* input bytes per wave of b200sdr_batch_host (two wave buffers)   */
 
 struct AudioFifo {
     float *d_buf = nullptr;   /* device FIFO storage: valid floats are d_buf[head .. head + count)  */
@@ -234,7 +221,7 @@ bool make_tc_tensor_map(CUtensorMap *map, const uint8_t *iq_dev, uint32_t n_capt
     memset(map, 0, sizeof *map);
     const tensor_map_encode_fn enc = tensor_map_encoder();
     const uint64_t rows = len_bytes / B200_TC_ROW_BYTES;
-    if (!enc || rows == 0 || getenv("B200SDR_TC_NO_TMA")) return false;
+    if (!enc || rows == 0) return false;
     const cuuint64_t dims[3] = {B200_TC_ROW_BYTES, rows, n_captures};
     const cuuint64_t strides[2] = {B200_TC_ROW_BYTES, len_bytes};
     const cuuint32_t box[3] = {64, B200_TC_ROWS, 1}, elem[3] = {1, 1, 1};
@@ -265,7 +252,6 @@ int launch_wbfm_tc_batch(b200sdr_ctx *ctx, const uint8_t *iq_dev, uint32_t n_cap
     p.b_image = ctx->d_tc_image;
     p.error = ctx->d_tc_error;
     p.dbg_acc = dbg_acc;
-    { const char *e = getenv("B200SDR_TC_DEBUG"); p.dbg_flags = e ? (uint32_t)atoi(e) : 0u; } /* timing experiments (tools/tc_check.py) */
     /* TMA for every tile made of whole rows; the tile with a capture's ragged last row (length not a multiple of 320
      * bytes) is filled with bounds-checked cp.async by the same kernel */
     alignas(64) CUtensorMap tmap;
@@ -1077,7 +1063,7 @@ int32_t b200sdr_batch_host(b200sdr_ctx *ctx, uint32_t chains, const uint8_t *iq_
     if ((chains & B200SDR_CHAIN_WBFM) && !wbfm_audio_host) return B200SDR_FAIL;
     if ((chains & B200SDR_CHAIN_AM) && !am_audio_host) return B200SDR_FAIL;
     DeviceGuard guard(ctx->device);
-    uint64_t per_wave = wave_bytes_target() / len_each;
+    uint64_t per_wave = kWaveBytes / len_each;
     if (per_wave < 1) per_wave = 1;
     if (per_wave > n_captures) per_wave = n_captures;
     const size_t wave_bytes = (size_t)per_wave * len_each;
@@ -1567,7 +1553,7 @@ int32_t b200sdr_host_alloc_pinned(b200sdr_ctx *ctx, uint64_t bytes, void **out_h
 {
     if (!ctx || !out_host) return B200SDR_FAIL;
     DeviceGuard guard(ctx->device);
-    CU(cudaHostAlloc(out_host, bytes ? bytes : 16, pinned_flags()));
+    CU(cudaHostAlloc(out_host, bytes ? bytes : 16, cudaHostAllocDefault));
     return B200SDR_OK;
 }
 int32_t b200sdr_host_free_pinned(b200sdr_ctx *ctx, void *host)

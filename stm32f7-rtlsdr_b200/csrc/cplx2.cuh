@@ -29,13 +29,10 @@
 #endif
 
 #if defined(__CUDA_ARCH__) && !defined(B200_EMULATED)
-#define B200_PACKED 1 /* real device code (inline PTX allowed) */
-#if !defined(B200_SCALAR_MATH) || !B200_SCALAR_MATH
-#define B200_PACKED_MATH 1 /* complex numbers as fp32x2 pairs; -DB200_SCALAR_MATH=1 is the A/B knob */
-#endif
+#define B200_PACKED 1 /* real device code (inline PTX allowed): complex numbers as fp32x2 pairs */
 #endif
 
-#ifdef B200_PACKED_MATH
+#ifdef B200_PACKED
 
 struct c2 { unsigned long long v; };
 
@@ -104,92 +101,26 @@ B200_DEV float c2_norm_acc(c2 a, float acc)
 
 /* ---- u8 I/Q -> exact float (u - 127.5) without an integer->float conversion.
  *
- * Form A (B200_CVT_FHADD = 0): PRMT drops the byte into mantissa bits [15:8] of 2^15 and 0x80 into
- * bits [7:0]: 0x47000080 | (u << 8) is the float 32768.5 + u exactly (ulp of bit 8 at 2^15 is 1), and
- * one FADD of -32896 leaves u - 127.5 exactly.  (The textbook 2^23 + u form cannot subtract
+ * Form A (the spectrum kernel and the cf32 conversion): PRMT drops the byte into mantissa bits [15:8] of 2^15
+ * and 0x80 into bits [7:0]: 0x47000080 | (u << 8) is the float 32768.5 + u exactly (ulp of bit 8 at 2^15 is 1),
+ * and one FADD of -32896 leaves u - 127.5 exactly.  (The textbook 2^23 + u form cannot subtract
  * 8388735.5 -- it is not representable.)  Per complex sample: 2 PRMT (half rate) + 1 FADD2.
- *
- * Form B (B200_CVT_FHADD = 1, sm_100 mixed-precision add, SASS FHADD): ONE PRMT builds the half2
- * (0x6400 | I, 0x6400 | Q) = (1024 + I, 1024 + Q) exactly, and add.rn.f32.f16 takes either half
- * straight from the register (R.H0 / R.H1 operand selector) and adds the fp32 constant -1151.5:
- * u - 127.5 exactly, one PRMT + 2 FHADD per complex sample.
  * `word` holds 4 bytes = 2 complex samples. */
-#ifndef B200_CVT_FHADD
-#define B200_CVT_FHADD 0
-#endif
 #define B200_U8_MAGIC 0x47000080u
 #define B200_U8_BIAS  (-32896.0f)
-#define B200_H2_MAGIC 0x64646464u
-#define B200_H2_BIAS  (-1151.5f)
-/* The two constants of the conversion, fetched once per kernel and passed to every conversion.
- * Form B wants each in ONE ordinary register: FHADD has no immediate / uniform-register form and PRMT
- * has one immediate slot (wanted for the selector); whenever ptxas can prove such a value uniform it
- * keeps it in a uniform register and re-materialises it with a MOV next to nearly every use (one extra
- * issue slot per conversion, seen in the SASS -- it even folds (%laneid >> 5) back to a constant).
- * So one thread parks them in two words of shared memory before the kernel's first barrier and every
- * thread loads them after it: a loaded value is just a register to ptxas
- * (`PRMT R, Rw, 0x4140, Rm` / `FHADD R, R.H1, Rb.reuse`, no MOVs). */
-struct cvt_k { float bias; uint32_t magic; };
-B200_DEV void b200_cvt_consts_store(volatile uint32_t *s2) /* one thread, before a __syncthreads() */
-{
-#if defined(B200_PACKED) && B200_CVT_FHADD
-    s2[0] = 0xC48FF000u; /* -1151.5f */
-    s2[1] = B200_H2_MAGIC;
-#else
-    (void)s2;
-#endif
-}
-B200_DEV cvt_k b200_cvt_consts_load(const volatile uint32_t *s2) /* every thread, after it */
-{
-    cvt_k k;
-#if defined(B200_PACKED) && B200_CVT_FHADD
-    k.bias = __uint_as_float(s2[0]);
-    k.magic = s2[1];
-#else
-    (void)s2;
-    k.bias = B200_U8_BIAS;
-    k.magic = B200_U8_MAGIC;
-#endif
-    return k;
-}
-#if defined(B200_PACKED) && B200_CVT_FHADD
-B200_DEV c2 b200_h2_to_c2(uint32_t h2, float bias) /* h2 = half2 (1024 + I, 1024 + Q) */
-{
-    float i, q;
-    asm("{ .reg .b16 lo, hi; mov.b32 {lo, hi}, %2; add.rn.f32.f16 %0, lo, %3; add.rn.f32.f16 %1, hi, %3; }"
-        : "=f"(i), "=f"(q) : "r"(h2), "f"(bias));
-    return c2_make(i, q);
-}
-#endif
 B200_DEV float b200_u8_to_f32(uint32_t word, int byte_idx) /* byte_idx compile-time 0..3 */
 {
     uint32_t sel = 0x7504u | ((uint32_t)byte_idx << 4);
     return __uint_as_float(__byte_perm(word, B200_U8_MAGIC, sel)) + B200_U8_BIAS;
 }
-B200_DEV c2 c2_from_u8_lo(uint32_t word, cvt_k k) /* bytes 0 (I) and 1 (Q); k = b200_cvt_consts_load() */
+B200_DEV c2 c2_from_u8_lo(uint32_t word) /* bytes 0 (I) and 1 (Q) */
 {
-#if defined(B200_PACKED) && B200_CVT_FHADD
-    return b200_h2_to_c2(__byte_perm(word, k.magic, 0x4140), k.bias);
-#else
-    (void)k;
     float i = __uint_as_float(__byte_perm(word, B200_U8_MAGIC, 0x7504));
     float q = __uint_as_float(__byte_perm(word, B200_U8_MAGIC, 0x7514));
     return c2_add(c2_make(i, q), c2_make(B200_U8_BIAS, B200_U8_BIAS));
-#endif
-}
-B200_DEV c2 c2_from_u8_hi(uint32_t word, cvt_k k) /* bytes 2 (I) and 3 (Q) */
-{
-#if defined(B200_PACKED) && B200_CVT_FHADD
-    return b200_h2_to_c2(__byte_perm(word, k.magic, 0x4342), k.bias);
-#else
-    (void)k;
-    float i = __uint_as_float(__byte_perm(word, B200_U8_MAGIC, 0x7524));
-    float q = __uint_as_float(__byte_perm(word, B200_U8_MAGIC, 0x7534));
-    return c2_add(c2_make(i, q), c2_make(B200_U8_BIAS, B200_U8_BIAS));
-#endif
 }
 
-/* Form C (the FIR kernels, B200_FIR_RAWU8 = 1): NO conversion arithmetic.  PRMT drops the byte into bits
+/* Form C (the FIR kernels): NO conversion arithmetic.  PRMT drops the byte into bits
  * [23:16] of an otherwise zero word.  Read as a float that is u * 2^-133 EXACTLY for every u in 0..255:
  * u < 128 is the subnormal (u << 16) * 2^-149, u >= 128 has exponent field 1 and is
  * 2^-126 (1 + (u - 128) / 128) -- the subnormal / normal boundary is seamless, and FFMA2 (no .ftz)
@@ -198,9 +129,6 @@ B200_DEV c2 c2_from_u8_hi(uint32_t word, cvt_k k) /* bytes 2 (I) and 3 (Q) */
  * becomes one constant per OUTPUT instead of one add per INPUT sample: an accumulator is started at
  * -127.5 * sum(h) instead of 0 (wbfm.cuh / am.cuh).  The FP32 pipe, which bounds those kernels, then sees
  * only the FIR's own FMAs; the two PRMTs run on the integer pipe. */
-#ifndef B200_FIR_RAWU8
-#define B200_FIR_RAWU8 1
-#endif
 #define B200_U8RAW_LOG2 133
 B200_DEV c2 c2_u8raw_lo(uint32_t word) /* bytes 0 (I) and 1 (Q) -> (I, Q) * 2^-133 */
 {
@@ -210,12 +138,5 @@ B200_DEV c2 c2_u8raw_hi(uint32_t word) /* bytes 2 (I) and 3 (Q) */
 {
     return c2_make(__uint_as_float(__byte_perm(word, 0u, 0x4244)), __uint_as_float(__byte_perm(word, 0u, 0x4344)));
 }
-#if B200_FIR_RAWU8
-#define B200_FIR_X_LO(word, k) c2_u8raw_lo(word)
-#define B200_FIR_X_HI(word, k) c2_u8raw_hi(word)
-#else
-#define B200_FIR_X_LO(word, k) c2_from_u8_lo(word, k)
-#define B200_FIR_X_HI(word, k) c2_from_u8_hi(word, k)
-#endif
 
 #endif /* B200_CPLX2_CUH */

@@ -1,16 +1,17 @@
 /*
- * fft32.cuh -- 32-point complex FFT held entirely in one thread's registers.
+ * fft32.cuh -- the stages of a 32-point complex FFT held entirely in one thread's registers.
  *
  * Radix-2 decimation in time, forward transform X[k] = sum_n x[n] e^{-2 pi i k n / 32}.
- * The caller places x[bitrev5(i)] in slot i (a compile-time permutation of registers, free);
- * results come out in natural order.  Built from the packed-complex primitives of cplx2.cuh:
+ * Slot i holds x[bitrev5(i)] (a compile-time permutation of registers, free); after the stages
+ * of length 2, 4, .., 32 slot i holds X[i].  Built from the packed-complex primitives of cplx2.cuh:
  *   trivial twiddles (1, -j)   46 butterflies x 2 FADD2
  *   general twiddles           34 butterflies x 3 FFMA2   (X = a + W b: 2, Y = 2a - X: 1)
  * = 194 FP32x2 instructions per transform (388 fp32 lane-operations).
  *
- * The 1024-point transform of the spectrum chain is two of these (32 x 32 "four-step"), the
- * planned CMSIS shape being arm_cfft_f32 with arm_cfft_sR_f32_len1024 (reference
- * CMSIS/core/arm_math.h:2149, arm_const_structs.h:55 -- declared, never called).
+ * The 1024-point transform of the spectrum chain is two of these (32 x 32 "four-step"; spectrum.cuh
+ * fuses the first stage of each with the window or the twiddles), the planned CMSIS shape being
+ * arm_cfft_f32 with arm_cfft_sR_f32_len1024 (reference CMSIS/core/arm_math.h:2149,
+ * arm_const_structs.h:55 -- declared, never called).
  */
 #ifndef B200_FFT32_CUH
 #define B200_FFT32_CUH
@@ -71,15 +72,5 @@ template <int LEN>
 struct b200_stage_k<LEN, LEN / 2> {
     B200_DEVM static void run(c2 (&)[32]) {}
 };
-
-/* in-register FFT: slot i holds x[bitrev5(i)] on entry, X[i] on exit */
-B200_DEV void b200_fft32(c2 (&v)[32])
-{
-    b200_stage_k<2, 0>::run(v);
-    b200_stage_k<4, 0>::run(v);
-    b200_stage_k<8, 0>::run(v);
-    b200_stage_k<16, 0>::run(v);
-    b200_stage_k<32, 0>::run(v);
-}
 
 #endif

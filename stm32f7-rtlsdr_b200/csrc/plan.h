@@ -43,12 +43,8 @@ struct SpectrumPlan {
     uint32_t frames, frames_per_warp, units_per_capture, grid;
     uint64_t total_units;
 };
-#ifndef B200_SPEC_FPW_FIXED
-#define B200_SPEC_FPW_FIXED 0 /* timing experiments only (tools/variants.list): this many frames per warp, always */
-#endif
 inline uint32_t spectrum_frames_per_warp(uint64_t frames)
 {
-    if (B200_SPEC_FPW_FIXED) return B200_SPEC_FPW_FIXED;
     uint64_t fpw = ceil_div(frames, kSpecWarpsToFill);
     if (fpw < 1) fpw = 1;
     if (fpw > kSpecMaxFramesPerWarp) fpw = kSpecMaxFramesPerWarp;

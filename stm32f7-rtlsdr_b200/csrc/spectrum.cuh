@@ -16,8 +16,7 @@
  *   power:            acc[k2] += |X|^2                          32 bins per lane, in registers
  * The 32 window values and 32 twiddles a lane needs never change, so they are staged through shared
  * memory once per CTA and then held in registers (250 registers, 2 CTAs of 4 warps per SM): the only
- * shared-memory traffic per frame is the transpose (DESIGN.md 5.1 has the A/B measurements; the
- * compile-time knobs below are the A/B switches of those measurements, defaults = shipped).
+ * shared-memory traffic per frame is the transpose (DESIGN.md 5.1 has the measurements behind these choices).
  * Work unit = (capture, 4 x frames_per_warp consecutive frames).  A warp walks `frames_per_warp`
  * consecutive frames (hop 512) and keeps the 32 x 32 bin sums in registers; the four warps of the unit are
  * then added in a fixed order and one 1024-float partial per UNIT goes to a workspace that
@@ -46,55 +45,25 @@
 
 #include "fft32.cuh"
 
-#ifndef B200_SPEC_MINB
-#define B200_SPEC_MINB 2 /* CTAs per SM the register allocation is tuned for (8 warps/SM, up to 255 registers) */
-#endif
-#ifndef B200_SPEC_PREFETCH
-#define B200_SPEC_PREFETCH 1 /* issue the loads of frame m+1 before the FFT of frame m */
-#endif
-#ifndef B200_SPEC_FUSE_WIN
-#define B200_SPEC_FUSE_WIN 1 /* window multiply folded into the first butterfly stage of pass 1 */
-#endif
-#ifndef B200_SPEC_MERGE_TW
-#define B200_SPEC_MERGE_TW 1 /* fold the inter-pass twiddles into the first butterfly stage of pass 2 */
-#endif
-#ifndef B200_SPEC_REUSE
-#define B200_SPEC_REUSE 0 /* keep the upper 16 sample words of frame m in registers as the lower 16 of frame m+1 */
-#endif
-#ifndef B200_SPEC_REGCONST
-#define B200_SPEC_REGCONST 3 /* bit 0: this lane's 32 twiddles, bit 1: its 32 window values live in registers for the
-                                whole kernel instead of being re-read from shared memory every frame (needs MINB <= 2) */
-#endif
-/* TIMING EXPERIMENTS ONLY (results are wrong when non-zero; tools/gpu_variants.sh): bit 0 no window
- * loads, bit 1 no twiddle loads, bit 2 no transpose, bit 3 no global loads */
-#ifndef B200_SPEC_EXPERIMENT
-#define B200_SPEC_EXPERIMENT 0
-#endif
+#define B200_SPEC_MINB 2 /* CTAs per SM the register allocation is tuned for (8 warps/SM, up to 255 registers): the
+                            lane's 32 twiddles and 32 window values stay in registers for the whole kernel */
 #define B200_SPEC_WARPS 4
 #define B200_SPEC_THREADS (32 * B200_SPEC_WARPS)
-#ifndef B200_SPEC_XP
 #define B200_SPEC_XP 34 /* transpose tile row pitch in complex elements: 64-bit accesses conflict-free.
                            34 (even): rows are 16-byte aligned and are read back with 128-bit loads, also conflict-free */
-#endif
 #define B200_SPEC_WP 36 /* window row pitch in floats */
 
 /* shared memory carve-up (bytes) */
 #define B200_SPEC_SMEM_WIN 0
 #define B200_SPEC_SMEM_TW (32 * B200_SPEC_WP * 4)
 #define B200_SPEC_SMEM_XP (B200_SPEC_SMEM_TW + 32 * 32 * 8)
-#define B200_SPEC_SMEM_CVT (B200_SPEC_SMEM_XP + B200_SPEC_WARPS * 32 * B200_SPEC_XP * 8) /* u32 [2]: conversion constants */
-#define B200_SPEC_SMEM_BYTES (B200_SPEC_SMEM_CVT + 16)
+#define B200_SPEC_SMEM_SCHED (B200_SPEC_SMEM_XP + B200_SPEC_WARPS * 32 * B200_SPEC_XP * 8) /* u32 [4]: [2] next unit, [3] last CTA */
+#define B200_SPEC_SMEM_BYTES (B200_SPEC_SMEM_SCHED + 16)
 
 #ifdef B200_EMULATED
 #define B200_DYN_SMEM(name) unsigned char *name = EMU_DYN_SMEM
 #else
 #define B200_DYN_SMEM(name) extern __shared__ __align__(1024) unsigned char name[]
-#endif
-
-#if B200_SPEC_EXPERIMENT & 8
-#define B200_SPEC_LOAD(ptr) ((uint32_t)(uintptr_t)(ptr) * 2654435761u >> 16)
-#else
-#define B200_SPEC_LOAD(ptr) ((uint32_t)__ldg(ptr))
 #endif
 
 struct SpectrumParams {
@@ -138,39 +107,26 @@ __global__ void __launch_bounds__(B200_SPEC_THREADS, B200_SPEC_MINB) k_spectrum(
             s_win[t * B200_SPEC_WP + 2 * bi + h] = __ldg(p.window + i);
         }
         float2 w = __ldg(p.twiddle + ((t * j) & 1023));
-#if B200_SPEC_MERGE_TW
         /* pair layout: [e][lane] = (W^{e lane}, W^{(e+16) lane}), e = 0..15: one 16-byte load feeds a
          * first-stage butterfly of pass 2 (elements e and e+16 of lane's column) */
         s_tw[((j & 15) * 32 + t) * 2 + (j >> 4)] = c2_make(w.x, w.y);
-#else
-        s_tw[j * 32 + t] = c2_make(w.x, w.y);
-#endif
     }
-    uint32_t *s_cvt = reinterpret_cast<uint32_t *>(smem + B200_SPEC_SMEM_CVT);
-    if (tid == 0) b200_cvt_consts_store(s_cvt);
+    uint32_t *s_sched = reinterpret_cast<uint32_t *>(smem + B200_SPEC_SMEM_SCHED);
     __syncthreads();
-    const cvt_k cb = b200_cvt_consts_load(s_cvt);
 
     const float *my_win = s_win + lane * B200_SPEC_WP;
-#if B200_SPEC_EXPERIMENT & 3
-    const float fake_w = my_win[0] + 0.5f;
-#endif
-#if B200_SPEC_REGCONST & 1
     float4 r_tw[16];
 #pragma unroll
     for (int i = 0; i < 16; ++i) r_tw[i] = *reinterpret_cast<const float4 *>(s_tw + (b200_bitrev5(2 * i) * 32 + lane) * 2);
-#endif
-#if B200_SPEC_REGCONST & 2
     float4 r_win[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) r_win[i] = *reinterpret_cast<const float4 *>(my_win + 4 * i);
-#endif
 
     float *s_red = reinterpret_cast<float *>(smem + B200_SPEC_SMEM_XP); /* [warp][1024], pitch 32*XP*2 floats */
     uint32_t unit_g = blockIdx.x;
     while (unit_g < p.total_units) {
     /* ask for the next unit now; the answer is read after this unit's barriers */
-    if (tid == 0) s_cvt[2] = gridDim.x + atomicAdd(p.unit_counter, 1u);
+    if (tid == 0) s_sched[2] = gridDim.x + atomicAdd(p.unit_counter, 1u);
     const uint32_t capture = unit_g / p.units_per_capture;
     const uint32_t warp_global = (unit_g - capture * p.units_per_capture) * B200_SPEC_WARPS + (uint32_t)warp;
     const uint32_t m_begin = warp_global * p.frames_per_warp;
@@ -186,101 +142,60 @@ __global__ void __launch_bounds__(B200_SPEC_THREADS, B200_SPEC_MINB) k_spectrum(
      * so no warp ever waits on HBM/L2 latency with only two warps per scheduler resident */
     const unsigned short *src0 = reinterpret_cast<const unsigned short *>(cap) + (uint32_t)lane;
     uint32_t raw[32];
-    if (B200_SPEC_PREFETCH && m_begin < m_end) {
+    if (m_begin < m_end) {
 #pragma unroll
-        for (int j = 0; j < 32; ++j) raw[j] = B200_SPEC_LOAD(src0 + (uint64_t)m_begin * 512u + 32 * j);
+        for (int j = 0; j < 32; ++j) raw[j] = __ldg(src0 + (uint64_t)m_begin * 512u + 32 * j);
     }
     for (uint32_t m = m_begin; m < m_end; ++m) {
         c2 v[32];
-        if (!B200_SPEC_PREFETCH) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) raw[j] = B200_SPEC_LOAD(src0 + (uint64_t)m * 512u + 32 * j);
-        }
         /* convert, window and first DIT stage of pass 1 in one go: butterfly i takes samples
          * e = bitrev5(2 i) and e + 16:  X = a wa + b wb,  Y = a wa - b wb  (3 packed ops) */
 #pragma unroll
         for (int i2 = 0; i2 < 8; ++i2) {
-#if B200_SPEC_EXPERIMENT & 1
-            const float4 w4 = make_float4(fake_w, fake_w, fake_w, fake_w);
-#elif B200_SPEC_REGCONST & 2
             const float4 w4 = r_win[i2];
-#else
-            const float4 w4 = *reinterpret_cast<const float4 *>(my_win + 4 * i2);
-#endif
             const float wv[4] = {w4.x, w4.y, w4.z, w4.w};
 #pragma unroll
             for (int ii = 0; ii < 2; ++ii) {
                 const int i = 2 * i2 + ii, e = b200_bitrev5(2 * i);
-                const c2 pa = c2_scale(c2_from_u8_lo(raw[e], cb), wv[2 * ii]);
-#if B200_SPEC_FUSE_WIN
-                const c2 b = c2_from_u8_lo(raw[e + 16], cb);
+                const c2 pa = c2_scale(c2_from_u8_lo(raw[e]), wv[2 * ii]);
+                const c2 b = c2_from_u8_lo(raw[e + 16]);
                 v[2 * i] = c2_fma_s(b, wv[2 * ii + 1], pa);
                 v[2 * i + 1] = c2_fma_s(b, -wv[2 * ii + 1], pa);
-#else
-                const c2 pb = c2_scale(c2_from_u8_lo(raw[e + 16], cb), wv[2 * ii + 1]);
-                v[2 * i] = c2_add(pa, pb);
-                v[2 * i + 1] = c2_sub(pa, pb);
-#endif
             }
         }
-        if (B200_SPEC_PREFETCH && m + 1 < m_end) {
+        if (m + 1 < m_end) {
             const unsigned short *src = src0 + (uint64_t)(m + 1) * 512u;
-#if B200_SPEC_REUSE
-            /* samples t + 32 (j + 16) of frame m are samples t + 32 j of frame m + 1 (hop 512) */
 #pragma unroll
-            for (int j = 0; j < 16; ++j) raw[j] = raw[j + 16];
-#pragma unroll
-            for (int j = 16; j < 32; ++j) raw[j] = B200_SPEC_LOAD(src + 32 * j);
-#else
-#pragma unroll
-            for (int j = 0; j < 32; ++j) raw[j] = B200_SPEC_LOAD(src + 32 * j);
-#endif
+            for (int j = 0; j < 32; ++j) raw[j] = __ldg(src + 32 * j);
         }
         b200_stage_k<4, 0>::run(v);
         b200_stage_k<8, 0>::run(v);
         b200_stage_k<16, 0>::run(v);
         b200_stage_k<32, 0>::run(v); /* v[k1] = Y[k1] */
-#if !B200_SPEC_MERGE_TW
-#pragma unroll
-        for (int k1 = 1; k1 < 32; ++k1) {
-            float wr, wi;
-            c2_get(s_tw[k1 * 32 + lane], wr, wi);
-            v[k1] = c2_cmul(v[k1], wr, wi);
-        }
-#endif
         /* transpose through the warp-private tile: row = k1 (the reader's lane), column = source lane t.
          * The barrier that keeps this frame's stores behind the previous frame's loads sits HERE, a whole
          * pass later than those loads, so it never waits on them. */
-#if !(B200_SPEC_EXPERIMENT & 4)
         __syncwarp();
 #pragma unroll
         for (int k1 = 0; k1 < 32; ++k1) s_xp[k1 * B200_SPEC_XP + lane] = v[k1];
         __syncwarp();
 #pragma unroll
-#if (B200_SPEC_XP % 2) == 0 && defined(B200_PACKED_MATH)
+#ifdef B200_PACKED
         for (int t = 0; t < 32; t += 2) {
             const float4 q = *reinterpret_cast<const float4 *>(s_xp + lane * B200_SPEC_XP + t);
             v[b200_bitrev5(t)] = c2_make(q.x, q.y);
             v[b200_bitrev5(t + 1)] = c2_make(q.z, q.w);
         }
-#else
+#else /* host emulation: scalar c2 */
         for (int t = 0; t < 32; ++t) v[b200_bitrev5(t)] = s_xp[lane * B200_SPEC_XP + t];
 #endif
-#endif
-#if B200_SPEC_MERGE_TW
         /* first DIT stage of pass 2 with the four-step twiddles folded in: slots (2i, 2i+1) hold the
          * elements e = bitrev5(2i) < 16 and e + 16 of this lane's column; X = Ta a + Tb b, Y = Ta a - Tb b
          * = 2 (Ta a) - X: 5 packed ops instead of 2 + 2 (twiddles) + 2 (butterfly) */
 #pragma unroll
         for (int i = 0; i < 16; ++i) {
             const int e = b200_bitrev5(2 * i);
-#if B200_SPEC_EXPERIMENT & 2
-            const float4 tw = make_float4(fake_w, fake_w, fake_w, fake_w);
-#elif B200_SPEC_REGCONST & 1
             const float4 tw = r_tw[i];
-#else
-            const float4 tw = *reinterpret_cast<const float4 *>(s_tw + (e * 32 + lane) * 2);
-#endif
             const c2 pa = (e == 0) ? v[2 * i] : c2_cmul(v[2 * i], tw.x, tw.y);
             const c2 x = c2_cfma(v[2 * i + 1], tw.z, tw.w, pa);
             v[2 * i + 1] = c2_two_a_minus(pa, x);
@@ -290,9 +205,6 @@ __global__ void __launch_bounds__(B200_SPEC_THREADS, B200_SPEC_MINB) k_spectrum(
         b200_stage_k<8, 0>::run(v);
         b200_stage_k<16, 0>::run(v);
         b200_stage_k<32, 0>::run(v); /* v[k2] = X[lane + 32 k2] */
-#else
-        b200_fft32(v); /* v[k2] = X[lane + 32 k2] */
-#endif
         if (EMA) {
             float wgt = p.ema_beta * exp2f((float)(p.frames - 1u - m) * p.ema_log2_decay);
 #pragma unroll
@@ -318,20 +230,20 @@ __global__ void __launch_bounds__(B200_SPEC_THREADS, B200_SPEC_MINB) k_spectrum(
         out[k] = s;
     }
     if (p.final_out) __threadfence(); /* the partial must be visible to whichever CTA finishes last */
-    unit_g = s_cvt[2];
-    __syncthreads(); /* the reduction buffer and s_cvt[2] are free again */
+    unit_g = s_sched[2];
+    __syncthreads(); /* the reduction buffer and s_sched[2] are free again */
     } /* units */
     /* the last CTA out leaves the hand-out counter at zero for the next launch (atomicInc wraps its own word) ... */
     if (tid == 0) {
         const bool last = atomicInc(p.unit_counter + 1, gridDim.x - 1u) == gridDim.x - 1u;
         if (last) p.unit_counter[0] = 0u;
-        s_cvt[3] = last ? 1u : 0u;
+        s_sched[3] = last ? 1u : 0u;
     }
     /* ... and, for a single capture of the streaming path, adds up the partials: out = scale * sum_i partial_i +
      * carry_scale * carry, units in fixed order -- k_spectrum_finalize without the extra launch */
     if (p.final_out) {
         __syncthreads();
-        if (s_cvt[3]) {
+        if (s_sched[3]) {
             __threadfence();
             /* a thread owns the bins 4 tid .. 4 tid + 3 and 512 + 4 tid ..; per bin the units are added in order (the same
              * sum as the separate kernel, bit for bit), with 128-bit loads and eight units at a time in flight -- one CTA

@@ -45,12 +45,8 @@
 #include "cplx2.cuh"
 #include "tma.cuh"
 
-#ifndef B200_FM_THREADS
 #define B200_FM_THREADS 128
-#endif
-#ifndef B200_FM_MINB
-#define B200_FM_MINB (B200_FM_THREADS == 128 ? 3 : 6)      /* CTAs per SM (shared memory: 71 KB / 37 KB per CTA) */
-#endif
+#define B200_FM_MINB 3                                     /* CTAs per SM (shared memory: 71 KB per CTA)        */
 #define B200_FM_WARPS (B200_FM_THREADS / 32)
 #define B200_FM_CHUNK 200                                  /* input samples per thread per tile      */
 #define B200_FM_OPT 20                                     /* stage-1 outputs per thread per tile    */
@@ -75,7 +71,7 @@
 #define B200_FM_SM_WSUM (B200_FM_SM_E + (B200_FM_HPAD + B200_FM_TILE_OUT + 16) * 4)     /* float [8]        */
 #define B200_FM_SM_TAILC (B200_FM_SM_WSUM + 32)                                         /* c2 [2][8]        */
 #define B200_FM_SM_YLASTC (B200_FM_SM_TAILC + 2 * 8 * 8)                                /* c2 [2]           */
-#define B200_FM_SM_BAR (B200_FM_SM_YLASTC + 16)                                         /* u64, u32 [2]     */
+#define B200_FM_SM_BAR (B200_FM_SM_YLASTC + 16)                                         /* u64 mbarrier, 8 spare */
 #define B200_FM_SMEM_BYTES (B200_FM_SM_BAR + 16)
 
 #ifndef B200_DYN_SMEM
@@ -156,23 +152,23 @@ B200_DEV void b200_fm_scatter(c2 x, c2 acc0, const float (&h)[40], c2 (&acc)[8],
 
 template <int Q>
 struct b200_fm_words {
-    B200_DEVM static void run(const uint4 *raw, cvt_k cb, c2 acc0, const float (&h)[40], c2 (&acc)[8], c2 (&out)[4])
+    B200_DEVM static void run(const uint4 *raw, c2 acc0, const float (&h)[40], c2 (&acc)[8], c2 (&out)[4])
     {
         const uint4 r = raw[Q];
-        b200_fm_scatter<8 * Q + 0>(B200_FIR_X_LO(r.x, cb), acc0, h, acc, out);
-        b200_fm_scatter<8 * Q + 1>(B200_FIR_X_HI(r.x, cb), acc0, h, acc, out);
-        b200_fm_scatter<8 * Q + 2>(B200_FIR_X_LO(r.y, cb), acc0, h, acc, out);
-        b200_fm_scatter<8 * Q + 3>(B200_FIR_X_HI(r.y, cb), acc0, h, acc, out);
-        b200_fm_scatter<8 * Q + 4>(B200_FIR_X_LO(r.z, cb), acc0, h, acc, out);
-        b200_fm_scatter<8 * Q + 5>(B200_FIR_X_HI(r.z, cb), acc0, h, acc, out);
-        b200_fm_scatter<8 * Q + 6>(B200_FIR_X_LO(r.w, cb), acc0, h, acc, out);
-        b200_fm_scatter<8 * Q + 7>(B200_FIR_X_HI(r.w, cb), acc0, h, acc, out);
-        b200_fm_words<Q + 1>::run(raw, cb, acc0, h, acc, out);
+        b200_fm_scatter<8 * Q + 0>(c2_u8raw_lo(r.x), acc0, h, acc, out);
+        b200_fm_scatter<8 * Q + 1>(c2_u8raw_hi(r.x), acc0, h, acc, out);
+        b200_fm_scatter<8 * Q + 2>(c2_u8raw_lo(r.y), acc0, h, acc, out);
+        b200_fm_scatter<8 * Q + 3>(c2_u8raw_hi(r.y), acc0, h, acc, out);
+        b200_fm_scatter<8 * Q + 4>(c2_u8raw_lo(r.z), acc0, h, acc, out);
+        b200_fm_scatter<8 * Q + 5>(c2_u8raw_hi(r.z), acc0, h, acc, out);
+        b200_fm_scatter<8 * Q + 6>(c2_u8raw_lo(r.w), acc0, h, acc, out);
+        b200_fm_scatter<8 * Q + 7>(c2_u8raw_hi(r.w), acc0, h, acc, out);
+        b200_fm_words<Q + 1>::run(raw, acc0, h, acc, out);
     }
 };
 template <>
 struct b200_fm_words<B200_FM_BLK / 8> {
-    B200_DEVM static void run(const uint4 *, cvt_k, c2, const float (&)[40], c2 (&)[8], c2 (&)[4]) {}
+    B200_DEVM static void run(const uint4 *, c2, const float (&)[40], c2 (&)[8], c2 (&)[4]) {}
 };
 
 #ifdef B200_EMULATED
@@ -225,7 +221,6 @@ __global__ void __launch_bounds__(B200_FM_THREADS, B200_FM_MINB) k_wbfm(FmParams
     c2 *s_tailc = reinterpret_cast<c2 *>(smem + B200_FM_SM_TAILC);
     c2 *s_ylastc = reinterpret_cast<c2 *>(smem + B200_FM_SM_YLASTC);
     uint64_t *s_bar = reinterpret_cast<uint64_t *>(smem + B200_FM_SM_BAR);
-    uint32_t *s_cvt = reinterpret_cast<uint32_t *>(smem + B200_FM_SM_BAR + 8); /* conversion constants (cplx2.cuh) */
 
     const int tid = (int)threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t capture = blockIdx.y;
@@ -244,13 +239,8 @@ __global__ void __launch_bounds__(B200_FM_THREADS, B200_FM_MINB) k_wbfm(FmParams
     /* taps and scan constants -> registers */
     float h[40];
 #pragma unroll
-#if B200_FIR_RAWU8
     for (int k = 0; k < 40; ++k) h[k] = taps->h1s[k];
     const c2 acc0 = c2_make(taps->bias_half, taps->bias_half);
-#else
-    for (int k = 0; k < 40; ++k) h[k] = taps->h1[k];
-    const c2 acc0 = c2_zero();
-#endif
     const float alpha = taps->alpha;
     const float a1 = 1.0f - alpha;
     float lane_pow = 1.0f; /* (a^OPT)^lane */
@@ -262,10 +252,8 @@ __global__ void __launch_bounds__(B200_FM_THREADS, B200_FM_MINB) k_wbfm(FmParams
     if (tid < 8) {
         float tr = 0.0f, ti = 0.0f;
         if (st_in) { tr = st_in->tail[2 * tid]; ti = st_in->tail[2 * tid + 1]; }
-#if B200_FIR_RAWU8
         /* first outputs of a capture / stream: x[n < 0] = 0 */
         if (seg == 0 && p.m_base == 0) tr = ti = taps->bias_head[tid];
-#endif
         s_tailc[8 + tid] = c2_make(tr, ti); /* tile 0 reads carry buffer 1 */
     }
     if (tid == 8) {
@@ -290,10 +278,8 @@ __global__ void __launch_bounds__(B200_FM_THREADS, B200_FM_MINB) k_wbfm(FmParams
         b200_mbar_init(s_bar, 1);
         b200_mbar_fence_init();
         if (my_tiles > 0) issue_tile(0);
-        b200_cvt_consts_store(s_cvt);
     }
     __syncthreads();
-    const cvt_k cb = b200_cvt_consts_load(s_cvt);
 
     for (uint32_t it = 0; it < my_tiles; ++it) {
         const uint32_t tile = t_begin + it;
@@ -321,14 +307,12 @@ __global__ void __launch_bounds__(B200_FM_THREADS, B200_FM_MINB) k_wbfm(FmParams
 #pragma unroll 1
         for (int blk = 0; blk < B200_FM_CHUNK / B200_FM_BLK; ++blk) {
             c2 out[4];
-            b200_fm_words<0>::run(reinterpret_cast<const uint4 *>(my_raw) + blk * (B200_FM_BLK / 8), cb, acc0, h, acc, out);
-#if B200_FIR_RAWU8
+            b200_fm_words<0>::run(reinterpret_cast<const uint4 *>(my_raw) + blk * (B200_FM_BLK / 8), acc0, h, acc, out);
             /* outputs 8.. of the chunk (blocks 2..) lived in this thread only: they hold one half of the offset, add
              * the other; outputs 0..7 get theirs from the previous thread's tails */
             const c2 fix = blk >= 2 ? acc0 : c2_zero();
 #pragma unroll
             for (int q = 0; q < 4; ++q) out[q] = c2_add(out[q], fix);
-#endif
 #pragma unroll
             for (int q = 0; q < 4; ++q) park[4 * blk + q] = out[q];
             /* local outputs 4..11 of this block are 0..7 of the next */

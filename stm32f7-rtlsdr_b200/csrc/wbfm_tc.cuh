@@ -123,7 +123,7 @@ struct FmTcParams {
     const uint8_t *b_image;  /* B200_TC_B_BYTES: the B operand as it lies in shared memory                      */
     uint32_t *error;         /* device word, 0 = ok; else which bounded wait expired                            */
     int32_t *dbg_acc;        /* optional [128][112]: raw accumulators of tile 0 of capture 0 (tests)            */
-    uint32_t dbg_flags;      /* timing experiments only: 1 = producer copies nothing, 2 = epilogue computes nothing */
+    uint32_t dbg_flags;      /* unused, zero: no kernel reads it; the host emulation harness of tests/emu still sets it */
 };
 
 #ifdef B200_EMULATED
@@ -466,7 +466,6 @@ B200_DEV bool b200_tc_epilogue_group(const FmTcParams &p, uint32_t n_items, uint
             const FmTcTile t = b200_tc_tile(p, w, tile, it);
             float e[B200_TC_OPR];
             if (!take(w, t, n, e, s_tot + (n % 3u) * 128)) return false;
-            if (p.dbg_flags & 2u) continue;
             b200_tc_epi_sync(grp); /* the group's row totals of tile n and its e[] of its previous tile are complete */
             if (have_pend) b200_tc_phase_c(p, pend_capture, pend_t, et, s_e_grp + (grp * 2 + ((pend_n >> 1) & 1u)) * B200_TC_EBUF);
             /* tile n - 1 is the other group's: its phase B (hence its row totals and its e[]) must be done.  Always waited
@@ -494,7 +493,7 @@ B200_DEV bool b200_tc_epilogue_group(const FmTcParams &p, uint32_t n_items, uint
             pend_n = n;
         }
     }
-    if (have_pend && !(p.dbg_flags & 2u)) { /* drain: the audio of the group's last tile */
+    if (have_pend) { /* drain: the audio of the group's last tile */
         b200_tc_epi_sync(grp);
         b200_tc_phase_c(p, pend_capture, pend_t, et, s_e_grp + (grp * 2 + ((pend_n >> 1) & 1u)) * B200_TC_EBUF);
     }
@@ -602,9 +601,7 @@ __global__ void __launch_bounds__(B200_TC_THREADS, 1) k_wbfm_tc(FmTcParams p)
                 if (!b200_tc_wait(bar_tfull + stage, phase ^ 1u, s_abort)) { ok = false; break; } /* MMAs of the tile two back done */
                 const uint32_t a_stage = a_base + stage * B200_TC_A_STAGE;
                 const int32_t R0 = (int32_t)(tile * B200_TC_ROWS);
-                if (p.dbg_flags & 1u) {
-                    if (lane == 0) b200_tc_arrive(bar_full + stage);
-                } else if (tile < p.manual_from_tile) {
+                if (tile < p.manual_from_tile) {
                     if (lane == 0) {
                         b200_tc_arrive_expect_tx(bar_full + stage, B200_TC_TX_BYTES);
 #pragma unroll
@@ -649,10 +646,8 @@ __global__ void __launch_bounds__(B200_TC_THREADS, 1) k_wbfm_tc(FmTcParams p)
                     if (!b200_tc_wait(bar_tempty + stage, phase ^ 1u, s_abort)) { fail = 3; break; }
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     const uint32_t a_stage = a_base + stage * B200_TC_A_STAGE;
-                    const int ksteps = (p.dbg_flags >> 8) ? (int)(p.dbg_flags >> 8) : B200_TC_KSTEPS; /* timing experiments */
 #pragma unroll
                     for (int ks = 0; ks < B200_TC_KSTEPS; ++ks) {
-                        if (ks >= ksteps) break;
                         const uint64_t da = b200_tc_desc(a_stage + (uint32_t)((ks >> 1) * B200_TC_A_BOX + (ks & 1) * 32));
                         const uint64_t db = b200_tc_desc(b_base + (uint32_t)((ks >> 1) * B200_TC_B_BOX + (ks & 1) * 32));
                         b200_tc_mma(tmem + stage * B200_TC_ACC_COLS, da, db, ks > 0 ? 1u : 0u);
@@ -712,7 +707,6 @@ __global__ void __launch_bounds__(B200_TC_THREADS, 1) k_wbfm_tc(FmTcParams p)
 #pragma unroll
                 for (int c = 0; c < B200_TC_SLICE_COLS; ++c) p.dbg_acc[row * B200_TC_N + c] = (int32_t)d0[c];
             }
-            if (p.dbg_flags & 2u) return true;
             if (t.tile == 0) b200_tc_phase_a<true>(p, w, t, lo, d0, row, e, s_tot);
             else b200_tc_phase_a<false>(p, w, t, lo, d0, row, e, s_tot);
             return true;

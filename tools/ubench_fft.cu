@@ -1,5 +1,5 @@
 // ubench_fft.cu -- what does the spectrum kernel's OWN instruction stream cost when nothing but the
-// FP32 pipe is in the way?  Runs csrc/fft32.cuh's register FFT-32 (the body of k_spectrum, 194 packed
+// FP32 pipe is in the way?  Runs a register FFT-32 of csrc/fft32.cuh's stages (the body of k_spectrum, 194 packed
 // ops) in a loop, alone and together with the other per-frame ingredients (u8 conversion PRMTs, the
 // transpose through shared memory), at the kernel's occupancy (128-thread CTAs, 2 / 3 / 4 per SM).
 // Prints FP32-pipe cycles per FFT-32 per scheduler against the nominal 2 cycles per packed op.
@@ -10,6 +10,15 @@
 #include "../stm32f7-rtlsdr_b200/csrc/cplx2.cuh"
 #include "../stm32f7-rtlsdr_b200/csrc/fft32.cuh"
 
+/* in-register FFT: slot i holds x[bitrev5(i)] on entry, X[i] on exit */
+__device__ __forceinline__ void b200_fft32(c2 (&v)[32])
+{
+    b200_stage_k<2, 0>::run(v);
+    b200_stage_k<4, 0>::run(v);
+    b200_stage_k<8, 0>::run(v);
+    b200_stage_k<16, 0>::run(v);
+    b200_stage_k<32, 0>::run(v);
+}
 
 // MODE 0: FFT-32 only          1: + 32 u16 -> c2 conversions (2 PRMT + FADD2 each)
 // MODE 2: + transpose (32 STS.64 + 32 LDS.64, pitch 33)      3: all of it
@@ -25,15 +34,11 @@ __global__ void __launch_bounds__(128, MINB) k_fft(float *out, const uint32_t *w
         v[i] = c2_make(1e-3f * (float)(threadIdx.x + i), 2e-3f * (float)i);
         w[i] = words[(threadIdx.x + i) & 1023];
     }
-    __shared__ uint32_t s_cvt[2];
-    if (threadIdx.x == 0) b200_cvt_consts_store(s_cvt);
-    __syncthreads();
-    const cvt_k cb = b200_cvt_consts_load(s_cvt);
     for (int it = 0; it < iters; ++it) {
         if (MODE & 1) {
 #pragma unroll
             for (int i = 0; i < 32; ++i) {
-                v[i] = c2_add(v[i], c2_from_u8_lo(w[i], cb));
+                v[i] = c2_add(v[i], c2_from_u8_lo(w[i]));
                 w[i] += 0x0101u; /* keep the conversion loop-variant (one IADD per word) */
             }
         }
